@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W]                 # this repo's sm_100a kernels
     python bench.py --impl reference [--gpus N] [--steps K] [--warmup W] # the reference's path on the host CPU cores
+    python bench.py ... --dump-outputs DIR     # also write what the timed path returned in its last step as DIR/*.npy
 
 One "step" = one pass of the hot path over one batch of synthetic input = rendering this rank's shard of a
 512x512 head+torso clip (BASELINE config "May head+torso two-pass 512x512, 250 frames, 1xB200"; at N GPUs every
@@ -53,7 +54,30 @@ def parse():
     ap.add_argument("--no-train-ops", action="store_true", help="skip timing the training-side native ops beside the reference's kernels (SURVEY 8(f) rank 4)")
     ap.add_argument("--precision", default=os.environ.get("GFPP_BENCH_PRECISION", DEFAULT_PRECISION), choices=["fp32", "fp16", "bf16x3", "bf16", "robust"],
                     help="arithmetic of the head MLP GEMMs (marching/gather/compositing are fp32 in every mode)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the timed path returned in its last step as DIR/<name>.npy (at most ~56 MB)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+def dump_outputs(path, clip, stats, H, W):
+    """What the last timed step returned, so that two builds can be compared output for output on identical inputs:
+    clip [F, H*W, 3] (fp32 frames at N = 1, the gathered uint8 clip at N > 1) and stats [F, 4] (B_total, n_survivors, S, P
+    per frame).  A fixed, seeded sample of 2^21 clip values with their flat indices (24 MB), and up to 4 whole frames, at
+    most 32 MB of them: at most ~56 MB in all."""
+    import numpy as np
+    import torch
+    os.makedirs(path, exist_ok=True)
+    g = torch.Generator().manual_seed(0)
+    flat = clip.reshape(-1)
+    idx = torch.randint(0, flat.numel(), (min(flat.numel(), 1 << 21),), generator=g).sort().values
+    k = min(4, clip.shape[0], (32 << 20) // (clip[0].numel() * 4))
+    pick = torch.randperm(clip.shape[0], generator=g)[:k].sort().values
+    arrays = {"clip_sample": flat[idx.to(flat.device)].float(), "clip_sample_index": idx.double(),
+              "frames": clip[pick.to(clip.device)].float().reshape(k, H, W, 3), "frame_index": pick.double(), "stats": stats.double()}
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a.cpu().numpy())
 
 
 def peaks():
@@ -385,10 +409,13 @@ def _main(args, out):
     sync_all()
     ev0.record()
     for _ in range(args.steps):
-        step_device()
+        last = step_device()
     ev1.record()
     sync_all()
     clocks = sampler.stop() if rank == 0 else {}
+    if rank == 0 and args.dump_outputs:
+        # before the legs below reuse the clip buffer
+        dump_outputs(args.dump_outputs, last, torch.cat(stats_acc, 0)[-T:], H, W)
     ms = ev0.elapsed_time(ev1)
     tms = torch.tensor([ms], device=dev)
     if world > 1:
